@@ -15,7 +15,9 @@ iterations per window, solved states back), host <-> device copies inside the ti
 Extra keys of the same line: the other BASELINE configurations with the CPU port timed beside them (single cfg3 / cfg4
 windows, marginalisation, literal config 5), single-window latency, a heterogeneous batch, KLT, PnP, IMU pre-integration.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--windows W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--windows W] [--dump-outputs DIR]
+--dump-outputs DIR writes what the last timed step computed, as a caller of the batched GN step receives it
+(dump_outputs below), so that two builds run with the same arguments can be compared output for output.
 Multi-GPU: python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N (one rank per GPU;
 windows are independent, so there is no data-path collective: scaling is weak, NCCL carries only
 the start barrier and the max-over-ranks of the device time).
@@ -167,6 +169,24 @@ def run_reference(args):
     return 0
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, dx, costs):
+    """Writes the batched GN step's results as pvio_b200_batch_download returns them: dx.npy [windows, 15 N + M]
+    (the step of every window) and costs.npy [windows, 2] (cost at the state, cost at the candidate), float64.
+    If all windows exceed DUMP_BYTES, a fixed seeded sample of windows (ascending) is written instead, the same
+    rows for the same --windows."""
+    n = len(dx)
+    keep = np.arange(n)
+    per_window = dx.itemsize * dx.shape[1] + costs.itemsize * costs.shape[1]
+    if n * per_window > DUMP_BYTES - 4096:          # room for the two .npy headers
+        keep = np.sort(np.random.default_rng(0).choice(n, (DUMP_BYTES - 4096) // per_window, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "dx.npy"), np.ascontiguousarray(dx[keep], dtype=np.float64))
+    np.save(os.path.join(out_dir, "costs.npy"), np.ascontiguousarray(costs[keep], dtype=np.float64))
+
+
 def time_call(fn, reps, warm=1):
     for _ in range(warm):
         fn()
@@ -240,6 +260,8 @@ def run_gpu(args):
     ms = ba.timer_stop()
     barrier()
     launches = ba.kernel_launches - l0
+    if args.dump_outputs and rank == 0:         # before the e2e calls below replace the batch on the device
+        dump_outputs(args.dump_outputs, *ba.batch_download(W, 15 * N + M))
     stage_ms, lin_ms, schur_ms = ba.last_kernel_ms(1), ba.last_kernel_ms(2), ba.last_kernel_ms(3)
     clocks = sampler.stop() if sampler else None
     ms_max = allmax(ms)
@@ -585,7 +607,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--windows", type=int, default=4096, help="independent cfg2 windows per GPU per step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's dx and costs as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         return run_reference(args)
     return run_gpu(args)
