@@ -3,9 +3,7 @@
 // one pipeline (frame-major table -> linearise -> Schur -> solve -> back-substitution / candidate), in fp32
 // Jacobians for visual-only windows and fp64 for windows with motion states.
 #include <algorithm>
-#include <chrono>
 #include <cmath>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <numeric>
@@ -27,8 +25,10 @@ int fail(Handle *h, int code, const char *what, cudaError_t e) {
     return code;
 }
 
+// (re)allocates b: n zeroed elements on the device and, if pinned, in pinned host staging; what b held is freed first
 template <typename T>
 static int alloc(Handle *h, DevBuf<T> &b, size_t n, bool pinned) {
+    b = DevBuf<T>();
     b.n = n;
     if (n == 0) return 0;
     CK(h, cudaMalloc(&b.d, n * sizeof(T)));
@@ -40,11 +40,15 @@ static int alloc(Handle *h, DevBuf<T> &b, size_t n, bool pinned) {
     return 0;
 }
 
-template <typename T>
-static void release(DevBuf<T> &b) {
-    if (b.d) cudaFree(b.d);
-    if (b.h) cudaFreeHost(b.h);
-    b.d = nullptr; b.h = nullptr; b.n = 0;
+SolveOpts solve_opts(const pvio_b200_options *opt) {
+    SolveOpts o;
+    if (opt) {
+        o.max_iter = opt->max_iterations;
+        if (opt->initial_trust_region_radius > 0) o.radius0 = opt->initial_trust_region_radius;
+        o.alias_bias = opt->alias_bias;
+        o.max_time = opt->max_time;
+    }
+    return o;
 }
 
 void drop_graphs(Handle *h) {
@@ -52,55 +56,87 @@ void drop_graphs(Handle *h) {
     h->graphs.clear();
 }
 
-static int ensure_inertial(Handle *h) {
-    if (h->have_inertial) return 0;
-    const size_t W = h->W, N = h->Ncap, dcap = 15 * N;
-    cudaStreamSynchronize(h->stream);
-    drop_graphs(h);                                 // the record array is reallocated below: pointers in cached graphs go stale
-    TRY(alloc(h, h->imu_idx, W * N * 2, true));
-    TRY(alloc(h, h->imu_data, W * N * kImuStride, true));
-    TRY(alloc(h, h->prior_frames, W * N, true));
-    TRY(alloc(h, h->prior_S, W * dcap * dcap, true));
-    TRY(alloc(h, h->prior_L, W * dcap * dcap, false));
-    TRY(alloc(h, h->prior_e, W * dcap, true));
-    TRY(alloc(h, h->prior_x0, W * N * kFrameStride, true));
-    // windows with motion states run the fp64 pipeline: h records of 8-byte elements
-    release(h->hs); release(h->jr); release(h->lm_w);
-    TRY(alloc(h, h->hs, 2 * W * N * (size_t)h->Mcap * 6 * sizeof(double), false));      // two buffer sets (LinBufs)
-    TRY(alloc(h, h->jr, 2 * W * N * (size_t)h->Mcap * 2 * sizeof(double), false));
-    TRY(alloc(h, h->lm_w, 2 * W * (size_t)h->Mcap * 2 * sizeof(double), false));
-    h->hs_double = true;
-    h->have_inertial = true;
+// The per-window input arrays: pack_window fills their pinned staging, upload_range copies it to the device.
+// f(m, n, g) is called for each array h->*m, with n elements per window and the array's group g, skipping the
+// groups the handle has not allocated.  The prior arrays are allocated with the inertial ones; they are a group of
+// their own because a device-resident prior is not uploaded.
+enum InputGroup { kVision, kInertial, kPrior, kPlanes };
+
+template <class F>
+static int for_each_input(const Handle *h, F f) {
+    const size_t N = h->Ncap, dcap = 15 * N;
+    TRY(f(&Handle::hdr, 1, kVision));
+    TRY(f(&Handle::cst, 1, kVision));
+    TRY(f(&Handle::obs, h->Kcap, kVision));
+    TRY(f(&Handle::lms, h->Mcap, kVision));
+    TRY(f(&Handle::rho, h->Mcap, kVision));
+    TRY(f(&Handle::frames, N * kFrameStride, kVision));
+    if (h->have_inertial) {
+        TRY(f(&Handle::imu_idx, N * 2, kInertial));
+        TRY(f(&Handle::imu_data, N * kImuStride, kInertial));
+        TRY(f(&Handle::prior_frames, N, kInertial));
+        TRY(f(&Handle::prior_S, dcap * dcap, kPrior));
+        TRY(f(&Handle::prior_e, dcap, kPrior));
+        TRY(f(&Handle::prior_x0, N * kFrameStride, kPrior));
+    }
+    if (h->have_planes) {
+        TRY(f(&Handle::plane_param, (size_t)h->Pcap * 4, kPlanes));
+        TRY(f(&Handle::pt_plane, h->Tcap, kPlanes));
+        TRY(f(&Handle::pt_begin, h->Tcap + 1, kPlanes));
+        TRY(f(&Handle::pt_frame, h->Ocap, kPlanes));
+        TRY(f(&Handle::pt_z, 2 * (size_t)h->Ocap, kPlanes));
+    }
     return 0;
 }
 
+static int alloc_inertial(Handle *h) {
+    const size_t W = h->W, N = h->Ncap, M = h->Mcap, dcap = 15 * N;
+    TRY(for_each_input(h, [&](auto m, size_t per, InputGroup g) {
+        return g == kInertial || g == kPrior ? alloc(h, h->*m, W * per, true) : 0;
+    }));
+    TRY(alloc(h, h->prior_L, W * dcap * dcap, false));
+    // windows with motion states run the fp64 pipeline: h records of 8-byte elements
+    TRY(alloc(h, h->hs, 2 * W * N * M * 6 * sizeof(double), false));      // two buffer sets (LinBufs)
+    TRY(alloc(h, h->jr, 2 * W * N * M * 2 * sizeof(double), false));
+    TRY(alloc(h, h->lm_w, 2 * W * M * 2 * sizeof(double), false));
+    h->hs_double = true;
+    return 0;
+}
+
+static int ensure_inertial(Handle *h) {
+    if (h->have_inertial) return 0;
+    cudaStreamSynchronize(h->stream);
+    drop_graphs(h);                                 // the record array is reallocated below: pointers in cached graphs go stale
+    h->have_inertial = true;                        // for_each_input visits the inertial arrays from here on
+    const int rc = alloc_inertial(h);
+    if (rc != 0) h->have_inertial = false;          // the next inertial window allocates again
+    return rc;
+}
+
 // Plane buffers grow on demand WITHOUT losing the slots already packed into the pinned staging area
-// (the device copies are refreshed by the next upload anyway).
+// (the device copies are refreshed by the next upload anyway).  The grown arrays replace the old ones only once all
+// of them are allocated, so a failed allocation leaves the handle as it was.
 static int ensure_planes(Handle *h, int T, int O) {
     if (h->have_planes && T <= h->Tcap && O <= h->Ocap) return 0;
-    const int Tn = std::max({T, h->Tcap, 256}), On = std::max({O, h->Ocap, 256 * 8});
     const size_t W = h->W;
     cudaStreamSynchronize(h->stream);
     drop_graphs(h);
-    DevBuf<double> pp; DevBuf<int32_t> tp, tb, tf; DevBuf<float> tz;
-    TRY(alloc(h, pp, W * h->Pcap * 4, true));
-    TRY(alloc(h, tp, W * Tn, true));
-    TRY(alloc(h, tb, W * (Tn + 1), true));
-    TRY(alloc(h, tf, W * On, true));
-    TRY(alloc(h, tz, W * On * 2, true));
-    if (h->have_planes) {
-        memcpy(pp.h, h->plane_param.h, sizeof(double) * W * h->Pcap * 4);
-        for (size_t i = 0; i < W; ++i) {
-            memcpy(tp.h + i * Tn, h->pt_plane.h + i * h->Tcap, sizeof(int32_t) * h->Tcap);
-            memcpy(tb.h + i * (Tn + 1), h->pt_begin.h + i * (h->Tcap + 1), sizeof(int32_t) * (h->Tcap + 1));
-            memcpy(tf.h + i * On, h->pt_frame.h + i * h->Ocap, sizeof(int32_t) * h->Ocap);
-            memcpy(tz.h + i * On * 2, h->pt_z.h + i * h->Ocap * 2, sizeof(float) * h->Ocap * 2);
-        }
-    }
-    release(h->plane_param); release(h->pt_plane); release(h->pt_begin); release(h->pt_frame); release(h->pt_z); release(h->pt_J);
-    h->plane_param = pp; h->pt_plane = tp; h->pt_begin = tb; h->pt_frame = tf; h->pt_z = tz;
-    TRY(alloc(h, h->pt_J, W * Tn * (6 * (size_t)h->Ncap + 2), false));      // device scratch of solve_kernel's plane block
-    h->Tcap = Tn; h->Ocap = On;
+    Handle g;                                       // capacities and arrays after the growth
+    g.W = h->W; g.Pcap = h->Pcap; g.have_planes = true;
+    g.Tcap = std::max({T, h->Tcap, 256}); g.Ocap = std::max({O, h->Ocap, 256 * 8});
+    TRY(for_each_input(&g, [&](auto m, size_t per, InputGroup grp) {
+        if (grp != kPlanes) return 0;
+        auto &to = g.*m;
+        const auto &from = h->*m;                   // empty before the first plane window
+        TRY(alloc(h, to, W * per, true));
+        const size_t old = from.n / W;              // old stride -> new stride, slot by slot
+        for (size_t i = 0; i < W && old > 0; ++i) memcpy(to.h + i * per, from.h + i * old, sizeof(*to.h) * old);
+        return 0;
+    }));
+    TRY(alloc(h, g.pt_J, W * g.Tcap * (6 * (size_t)h->Ncap + 2), false));      // device scratch of solve_kernel's plane block
+    for_each_input(&g, [&](auto m, size_t, InputGroup grp) { if (grp == kPlanes) (h->*m).swap(g.*m); return 0; });
+    h->pt_J.swap(g.pt_J);
+    h->Tcap = g.Tcap; h->Ocap = g.Ocap;
     h->have_planes = true;
     return 0;
 }
@@ -336,36 +372,15 @@ static int h2d(Handle *h, DevBuf<T> &b, size_t per, int w0, int n, cudaStream_t 
 // across the iterations of a solve: the frame-major table and Lambda = S^T S of the priors.
 static int upload_range(Handle *h, int w0, int n, cudaStream_t st) {
     if (n < 1 || w0 < 0 || w0 + n > h->W) return fail(h, PVIO_B200_EINVAL, "bad window range");
-    const size_t N = h->Ncap;
-    TRY(h2d(h, h->hdr, 1, w0, n, st));
-    TRY(h2d(h, h->cst, 1, w0, n, st));
-    TRY(h2d(h, h->obs, h->Kcap, w0, n, st));
-    TRY(h2d(h, h->lms, h->Mcap, w0, n, st));
-    TRY(h2d(h, h->rho, h->Mcap, w0, n, st));
-    TRY(h2d(h, h->frames, N * kFrameStride, w0, n, st));
+    const bool resident = w0 == 0 && n == 1 && h->prior_resident;     // a device-resident prior (marginalize_impl) is never re-uploaded
+    TRY(for_each_input(h, [&](auto m, size_t per, InputGroup g) {
+        return g == kPrior && resident ? 0 : h2d(h, h->*m, per, w0, n, st);
+    }));
     bool any_prior = false;
-    if (h->have_inertial) {
-        const size_t dcap = 15 * N;
-        TRY(h2d(h, h->imu_idx, N * 2, w0, n, st));
-        TRY(h2d(h, h->imu_data, N * kImuStride, w0, n, st));
-        TRY(h2d(h, h->prior_frames, N, w0, n, st));
-        if (!(w0 == 0 && n == 1 && h->prior_resident)) {     // a device-resident prior (marginalize_impl) is never re-uploaded
-            TRY(h2d(h, h->prior_S, dcap * dcap, w0, n, st));
-            TRY(h2d(h, h->prior_e, dcap, w0, n, st));
-            TRY(h2d(h, h->prior_x0, N * kFrameStride, w0, n, st));
-        }
-        for (int i = w0; i < w0 + n; ++i) any_prior |= h->hdr.h[i].n_prior > 0;
-        if (any_prior) {
-            prior_lambda_kernel<<<dim3(n, n < 64 ? 32 : 1), 256, 0, st>>>(h->hdr.d, h->prior_S.d, h->prior_L.d, h->Ncap, w0);
-            ++h->launches;
-        }
-    }
-    if (h->have_planes) {
-        TRY(h2d(h, h->plane_param, (size_t)h->Pcap * 4, w0, n, st));
-        TRY(h2d(h, h->pt_plane, h->Tcap, w0, n, st));
-        TRY(h2d(h, h->pt_begin, h->Tcap + 1, w0, n, st));
-        TRY(h2d(h, h->pt_frame, h->Ocap, w0, n, st));
-        TRY(h2d(h, h->pt_z, (size_t)h->Ocap * 2, w0, n, st));
+    if (h->have_inertial) for (int i = w0; i < w0 + n; ++i) any_prior |= h->hdr.h[i].n_prior > 0;
+    if (any_prior) {
+        prior_lambda_kernel<<<dim3(n, n < 64 ? 32 : 1), 256, 0, st>>>(h->hdr.d, h->prior_S.d, h->prior_L.d, h->Ncap, w0);
+        ++h->launches;
     }
     FobsArgs fa;
     fa.hdr = h->hdr.d; fa.obs = h->obs.d; fa.lms = h->lms.d; fa.fobs = h->fobs.d; fa.seg = h->seg.d;
@@ -460,7 +475,7 @@ static PipeArgs make_pipe_args(Handle *h, const StepCfg &c) {
     a.hdr = h->hdr.d; a.cst = h->cst.d; a.fobs = h->fobs.d; a.seg = h->seg.d; a.lms = h->lms.d;
     a.rho = h->rho.d; a.frames = h->frames.d; a.ctrl = h->ctrl.d; a.lm_scale = h->lm_scale.d; a.lm_aux = h->lm_aux.d;
     a.jr = h->jr.d; a.hs = h->hs.d; a.lm_w = h->lm_w.d; a.lm_msk = h->lm_msk.d;
-    a.Hred = h->Hred.d; a.Hdd = h->Hdd.d; a.gdir = h->gdir.d; a.gred = h->gred.d; a.cost_vis = h->cost_vis.d;
+    a.Hred = h->Hred.d; a.Hdd = h->Hdd; a.gdir = h->gdir; a.gred = h->gred; a.cost_vis = h->cost_vis;
     a.Ncap = h->Ncap; a.Mcap = h->Mcap; a.Kcap = h->Kcap;
     a.compute_scale = c.compute_scale; a.victim_only = 0; a.mu_override = c.mu; a.w0 = c.w0; a.loop = c.loop;
     return a;
@@ -564,7 +579,7 @@ static int run_linearize(Handle *h, int n, const StepCfg &c, const BatchShape &b
         for (auto &e : h->kev) CK(h, cudaEventCreate(&e));
     }
     const int slot = (h->kev_count % 256) * 3;
-    const bool timed = !h->capturing && !c.loop && !c.stream;   // stage times are a property of the plain batched step
+    const bool timed = !h->capturing && !c.loop && st == h->stream;   // stage times are a property of the plain batched step
     if (timed) CK(h, cudaEventRecord(h->kev[slot], st));
     TRY(launch_lin(h, n, c, b, loss, victim_only, false));
     if (timed) CK(h, cudaEventRecord(h->kev[slot + 1], st));
@@ -584,7 +599,7 @@ static int run_solve(Handle *h, int n, const StepCfg &c, const BatchShape &b) {
     SolveArgs a;
     memset(&a, 0, sizeof(a));
     a.hdr = h->hdr.d; a.cst = h->cst.d; a.frames = h->frames.d; a.ctrl = h->ctrl.d;
-    a.Hred = h->Hred.d; a.Hdd = h->Hdd.d; a.gdir = h->gdir.d; a.gred = h->gred.d; a.cost_vis = h->cost_vis.d;
+    a.Hred = h->Hred.d; a.Hdd = h->Hdd; a.gdir = h->gdir; a.gred = h->gred; a.cost_vis = h->cost_vis;
     a.imu_idx = h->imu_idx.d; a.imu_data = h->imu_data.d; a.alias_bias = c.alias_bias;
     a.prior_frames = h->prior_frames.d; a.prior_S = h->prior_S.d; a.prior_L = h->prior_L.d; a.prior_e = h->prior_e.d;
     a.prior_x0 = h->prior_x0.d;
@@ -618,7 +633,7 @@ static CostArgs make_cost_args(Handle *h, const StepCfg &c) {
     k.w0 = c.w0;
     k.ctrl = h->ctrl.d; k.acc = h->acc.d; k.frames_state = h->frames.d; k.rho_state = h->rho.d; k.rho_cand = h->rho_cand.d;
     k.Mcap = h->Mcap; k.loop = c.loop; k.apply = c.apply; k.beta = c.beta;
-    k.cost_vis = h->cost_vis.d; k.cost_stride = h->sys_set;
+    k.cost_vis = h->cost_vis; k.cost_stride = h->sys_set;
     return k;
 }
 
@@ -719,23 +734,24 @@ static int iteration_body(Handle *h, int n, const StepCfg &c, const BatchShape &
     return 0;
 }
 
-// The whole trust-region solve of the first n uploaded windows: init + max_iter (+ spare) identical bodies.  For the
-// latency path (few windows) the sequence is captured once into a CUDA graph keyed by (n, max_iter, flags) with
-// capacity-sized launch shapes, and replayed: ONE launch per solve, no device -> host traffic inside.
-static int run_solve_loop(Handle *h, int n, int max_iter, double max_time, double radius0, int alias_bias) {
+// The whole trust-region solve of the uploaded windows [w0, w0 + n) on stream st: init + max_iter (+ spare) identical
+// bodies.  For the latency path (few windows from 0 on the handle's stream) the sequence is captured once into a CUDA
+// graph keyed by (n, max_iter, flags) with capacity-sized launch shapes, and replayed: ONE launch per solve, no
+// device -> host traffic inside.
+static int run_solve_loop(Handle *h, int w0, int n, cudaStream_t st, const SolveOpts &o) {
     StepCfg c;
-    c.mu = -1.0; c.loop = 1; c.alias_bias = alias_bias; c.compute_scale = 0;
-    const bool graphable = n * 2 < h->sm_count;
-    const BatchShape b = batch_shape(h, 0, n, graphable);
-    const int bodies = max_iter + 2;                 // spare bodies absorb retries of a failed linear solve (mu *= 10)
-    init_ctrl_kernel<<<n, 32, 0, h->stream>>>(h->ctrl.d, 1e-8, radius0, max_iter, max_time, 0);
+    c.mu = -1.0; c.loop = 1; c.alias_bias = o.alias_bias; c.compute_scale = 0; c.w0 = w0; c.stream = st;
+    const bool graphable = w0 == 0 && st == h->stream && n * 2 < h->sm_count;
+    const BatchShape b = batch_shape(h, w0, n, graphable);
+    const int bodies = o.max_iter + 2;               // spare bodies absorb retries of a failed linear solve (mu *= 10)
+    init_ctrl_kernel<<<n, 32, 0, st>>>(h->ctrl.d, 1e-8, o.radius0, o.max_iter, o.max_time, w0);
     ++h->launches;
     LAUNCH_CK(h, "init_ctrl_kernel");
     if (!graphable) {
         for (int it = 0; it < bodies; ++it) TRY(iteration_body(h, n, c, b, it == 0));
         return 0;
     }
-    const Handle::GraphKey key(1, n, max_iter, (alias_bias ? 1 : 0) | (b.inertial ? 2 : 0) | (b.planes ? 4 : 0) | (h->hs_double ? 8 : 0) | (b.N << 4));
+    const Handle::GraphKey key(1, n, o.max_iter, (o.alias_bias ? 1 : 0) | (b.inertial ? 2 : 0) | (b.planes ? 4 : 0) | (h->hs_double ? 8 : 0) | (b.N << 4));
     auto it = h->graphs.find(key);
     if (it == h->graphs.end()) {
         if (h->graphs.size() >= 16) drop_graphs(h);
@@ -793,11 +809,20 @@ static int scatter_dx(Handle *h, int w0, int n, double *dx, int64_t dx_stride, d
     return 0;
 }
 
+// device -> host of the steps + control records of windows [w0, w0 + n) on stream st (async)
+static int download_dx_async(Handle *h, int w0, int n, cudaStream_t st) {
+    const size_t N = h->Ncap;
+    CK(h, cudaMemcpyAsync(h->dx_pose.h + (size_t)w0 * N * 15, h->dx_pose.d + (size_t)w0 * N * 15, sizeof(double) * N * 15 * n,
+                          cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(h->dx_lm.h + (size_t)w0 * h->Mcap, h->dx_lm.d + (size_t)w0 * h->Mcap, sizeof(double) * h->Mcap * n,
+                          cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(h->ctrl.h + w0, h->ctrl.d + w0, sizeof(WinCtrl) * n, cudaMemcpyDeviceToHost, st));
+    return 0;
+}
+
 static int download_dx(Handle *h, int n, double *dx, int64_t dx_stride, double *costs) {
     if (n < 1 || n > h->W) return fail(h, PVIO_B200_EINVAL, "bad window count");
-    CK(h, cudaMemcpyAsync(h->dx_pose.h, h->dx_pose.d, sizeof(double) * h->Ncap * 15 * n, cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaMemcpyAsync(h->dx_lm.h, h->dx_lm.d, sizeof(double) * h->Mcap * n, cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaMemcpyAsync(h->ctrl.h, h->ctrl.d, sizeof(WinCtrl) * n, cudaMemcpyDeviceToHost, h->stream));
+    TRY(download_dx_async(h, 0, n, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
     return scatter_dx(h, 0, n, dx, dx_stride, costs);
 }
@@ -819,15 +844,108 @@ static void fill_summary(const WinCtrl &c, pvio_b200_summary *sm) {
     sm->initial_cost = c.initial_cost; sm->final_cost = c.cost; sm->final_radius = c.radius; sm->final_mu = c.mu;
 }
 
-static void scatter_state(Handle *h, int i, double *frames, double *inv_depth) {
-    const int N = h->slot_N[i], M = h->slot_M[i];
-    if (frames) memcpy(frames, h->frames_out.h + (size_t)i * h->Ncap * kFrameStride, sizeof(double) * N * kFrameStride);
-    if (inv_depth) {
-        const double *r = h->rho_out.h + (size_t)i * h->Mcap;
-        const std::vector<int32_t> &perm = h->perm[i];
-        if (h->perm_identity[i]) memcpy(inv_depth, r, sizeof(double) * M);
-        else for (int lp = 0; lp < M; ++lp) inv_depth[perm[lp]] = r[lp];
+// downloaded states -> caller arrays (landmark order un-permuted) and summaries, windows [w0, w0 + n)
+static void scatter_states(Handle *h, int w0, int n, double *frames, int64_t frames_stride, double *inv_depth,
+                           int64_t inv_depth_stride, pvio_b200_summary *summaries) {
+    for (int i = w0; i < w0 + n; ++i) {
+        const int N = h->slot_N[i], M = h->slot_M[i];
+        if (frames)
+            memcpy(frames + (size_t)i * frames_stride, h->frames_out.h + (size_t)i * h->Ncap * kFrameStride, sizeof(double) * N * kFrameStride);
+        if (inv_depth) {
+            double *o = inv_depth + (size_t)i * inv_depth_stride;
+            const double *r = h->rho_out.h + (size_t)i * h->Mcap;
+            const std::vector<int32_t> &perm = h->perm[i];
+            if (h->perm_identity[i]) memcpy(o, r, sizeof(double) * M);
+            else for (int lp = 0; lp < M; ++lp) o[perm[lp]] = r[lp];
+        }
+        if (summaries) fill_summary(h->ctrl.h[i], &summaries[i]);
     }
+}
+
+// sub-batch schedule of the pipelined host paths: small batches first and last (the first upload and the last
+// kernels + download are the only parts of the pipeline that nothing overlaps), 512-window batches in between
+#ifndef PVIO_PIPE_STREAMS
+#define PVIO_PIPE_STREAMS 6
+#endif
+#ifndef PVIO_PIPE_CHUNK
+#define PVIO_PIPE_CHUNK 512
+#endif
+static constexpr int kPipeStreams = PVIO_PIPE_STREAMS;   // sub-batches in flight on the SMs at once (each alone is latency-bound: one wave)
+static std::vector<int> sub_batches(int n) {
+    std::vector<int> sizes;
+    if (n < 1024) { sizes.push_back(n); return sizes; }
+    int mid = n - 2 * (128 + 256);
+    sizes.push_back(128); sizes.push_back(256);
+    while (mid > 0) { const int m = std::min(PVIO_PIPE_CHUNK, mid); sizes.push_back(m); mid -= m; }
+    sizes.push_back(256); sizes.push_back(128);
+    return sizes;
+}
+
+static int ensure_pipeline_streams(Handle *h, int nsub) {
+    if (!h->stream_up) {
+        CK(h, cudaStreamCreateWithFlags(&h->stream_up, cudaStreamNonBlocking));
+        CK(h, cudaStreamCreateWithFlags(&h->stream_down, cudaStreamNonBlocking));
+    }
+    while ((int)h->ev_up.size() < nsub) {
+        cudaEvent_t a, b, c_;
+        CK(h, cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
+        CK(h, cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
+        CK(h, cudaEventCreateWithFlags(&c_, cudaEventDisableTiming));
+        h->ev_up.push_back(a); h->ev_done.push_back(b); h->ev_down.push_back(c_);
+    }
+    if (h->stream_c.empty()) {
+        h->stream_c.resize(kPipeStreams);
+        for (auto &st : h->stream_c) CK(h, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+        CK(h, cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
+    }
+    return 0;
+}
+
+// Upload, compute and download of windows [0, n) with HOST buffers.  Large batches are cut into sub-batches and
+// pipelined over three streams: host->device copy of sub-batch i+1 overlaps the kernels of sub-batch i and the
+// device->host copy of sub-batch i-1 (PCIe is full duplex), so the call costs max(copy, compute) instead of their sum.
+// The kernels of sub-batch i run on compute stream i % kPipeStreams (a sub-batch is at most one wave of CTAs, so alone
+// it runs at the latency of its kernel chain; several in flight fill the SMs); the windows of different sub-batches
+// share nothing on the device.  compute(w0, m, stream) and download(w0, m, stream) enqueue, scatter(w0, m) copies a
+// landed sub-batch to the caller while the GPU works on the later ones.
+template <class Compute, class Download, class Scatter>
+static int run_pipelined(Handle *h, int n, Compute compute, Download download, Scatter scatter) {
+    if (n < 1 || n > h->W) return fail(h, PVIO_B200_EINVAL, "bad window count");
+    const std::vector<int> sizes = sub_batches(n);
+    const int nsub = (int)sizes.size();
+    if (nsub == 1) {
+        TRY(upload(h, n));
+        TRY(compute(0, n, h->stream));
+        TRY(download(0, n, h->stream));
+        CK(h, cudaStreamSynchronize(h->stream));
+        return scatter(0, n);
+    }
+    std::vector<int> starts(nsub, 0);
+    for (int i = 1; i < nsub; ++i) starts[i] = starts[i - 1] + sizes[i - 1];
+    TRY(ensure_pipeline_streams(h, nsub));
+    CK(h, cudaEventRecord(h->ev_fork, h->stream));
+    CK(h, cudaStreamWaitEvent(h->stream_up, h->ev_fork, 0));
+    for (auto &sc : h->stream_c) CK(h, cudaStreamWaitEvent(sc, h->ev_fork, 0));
+    for (int i = 0; i < nsub; ++i) {
+        const int w0 = starts[i], m = sizes[i];
+        cudaStream_t sc = h->stream_c[i % kPipeStreams];
+        TRY(upload_range(h, w0, m, h->stream_up));
+        CK(h, cudaEventRecord(h->ev_up[i], h->stream_up));
+        CK(h, cudaStreamWaitEvent(sc, h->ev_up[i], 0));
+        TRY(compute(w0, m, sc));
+        CK(h, cudaEventRecord(h->ev_done[i], sc));
+        CK(h, cudaStreamWaitEvent(h->stream_down, h->ev_done[i], 0));
+        CK(h, cudaStreamWaitEvent(h->stream, h->ev_done[i], 0));      // later calls on the handle's stream see the result
+        TRY(download(w0, m, h->stream_down));
+        CK(h, cudaEventRecord(h->ev_down[i], h->stream_down));
+    }
+    h->n_uploaded = n;
+    for (int i = 0; i < nsub; ++i) {
+        CK(h, cudaEventSynchronize(h->ev_down[i]));
+        TRY(scatter(starts[i], sizes[i]));
+    }
+    CK(h, cudaStreamSynchronize(h->stream));
+    return 0;
 }
 
 }  // namespace pvio
@@ -859,10 +977,8 @@ int pvio_b200_create(int device, int max_windows, int max_frames, int max_landma
     CK(h, cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
     CK(h, cudaEventCreate(&h->ev0)); CK(h, cudaEventCreate(&h->ev1));
     const size_t W = h->W, N = h->Ncap, M = h->Mcap, K = h->Kcap, npc = N * (N + 1) / 2;
-    TRY(alloc(h, h->hdr, W, true)); TRY(alloc(h, h->cst, W, true));
-    TRY(alloc(h, h->obs, W * K, true)); TRY(alloc(h, h->lms, W * M, true));
+    TRY(for_each_input(h, [&](auto m, size_t per, InputGroup) { return alloc(h, h->*m, W * per, true); }));
     TRY(alloc(h, h->fobs, W * K, false)); TRY(alloc(h, h->seg, W * kSegTab, false));
-    TRY(alloc(h, h->rho, W * M, true)); TRY(alloc(h, h->frames, W * N * kFrameStride, true));
     TRY(alloc(h, h->ctrl, W, true));
     TRY(alloc(h, h->rho_cand, W * M, false)); TRY(alloc(h, h->frames_cand, W * N * kFrameStride, false));
     // the linearisation lives in two buffer sets (LinBufs, ba_types.h): everything below up to the reduced system is doubled
@@ -880,10 +996,10 @@ int pvio_b200_create(int device, int max_windows, int max_frames, int max_landma
         // multi-CTA-per-window mode (atomic accumulation) needs a single memset per launch
         const size_t n_sys = W * (npc * 36 + N * 36 + N * 6 + N * 6 + 1);
         TRY(alloc(h, h->Hred, 2 * n_sys, false));
-        h->Hdd.d = h->Hred.d + W * npc * 36; h->Hdd.n = 0;
-        h->gdir.d = h->Hdd.d + W * N * 36; h->gdir.n = 0;
-        h->gred.d = h->gdir.d + W * N * 6; h->gred.n = 0;
-        h->cost_vis.d = h->gred.d + W * N * 6; h->cost_vis.n = 0;
+        h->Hdd = h->Hred.d + W * npc * 36;
+        h->gdir = h->Hdd + W * N * 36;
+        h->gred = h->gdir + W * N * 6;
+        h->cost_vis = h->gred + W * N * 6;
         h->sys_set = n_sys;                                   // set 1 of each array lies n_sys elements behind set 0
     }
     TRY(alloc(h, h->acc, W * kAcc, true)); TRY(alloc(h, h->aux_cost, W, false));
@@ -926,15 +1042,6 @@ void pvio_b200_destroy(pvio_b200_handle hh) {
     resident_free(h);
     detect_free(h);
     fm_free(h);
-    release(h->hdr); release(h->cst); release(h->obs); release(h->lms); release(h->rho); release(h->frames);
-    release(h->fobs); release(h->seg); release(h->jr); release(h->lm_w); release(h->lm_msk); release(h->frames_out); release(h->rho_out); release(h->lm_v); release(h->valid); release(h->quality);
-    release(h->ctrl); release(h->rho_cand); release(h->frames_cand); release(h->lm_scale); release(h->lm_aux); release(h->hs);
-    release(h->dx_lm); release(h->dx_pose); release(h->pose_scale); release(h->v_pose); release(h->Hred);
-    release(h->acc); release(h->aux_cost);
-    release(h->Hfull); release(h->gfull);
-    release(h->imu_idx); release(h->imu_data); release(h->prior_frames); release(h->prior_S); release(h->prior_L);
-    release(h->prior_e); release(h->prior_x0);
-    release(h->pt_J); release(h->plane_param); release(h->pt_plane); release(h->pt_begin); release(h->pt_frame); release(h->pt_z);
     drop_graphs(h);
     for (auto &e : h->kev) cudaEventDestroy(e);
     cudaEventDestroy(h->ev0); cudaEventDestroy(h->ev1);
@@ -1016,30 +1123,13 @@ int pvio_b200_batch_replicate(pvio_b200_handle hh, int n) {
     Handle *h = reinterpret_cast<Handle *>(hh);
     if (!h) return PVIO_B200_EINVAL;
     if (n < 1 || n > h->W) return fail(h, PVIO_B200_EINVAL, "bad window count");
-    const size_t N = h->Ncap;
+    for_each_input(h, [&](auto m, size_t per, InputGroup) {
+        auto &b = h->*m;
+        for (int i = 1; i < n; ++i) memcpy(b.h + (size_t)i * per, b.h, sizeof(*b.h) * per);
+        return 0;
+    });
     for (int i = 1; i < n; ++i) {
-        h->hdr.h[i] = h->hdr.h[0]; h->cst.h[i] = h->cst.h[0];
-        memcpy(h->obs.h + (size_t)i * h->Kcap, h->obs.h, sizeof(ObsRec) * h->slot_K[0]);
-        memcpy(h->lms.h + (size_t)i * h->Mcap, h->lms.h, sizeof(LmRec) * h->slot_M[0]);
-        memcpy(h->rho.h + (size_t)i * h->Mcap, h->rho.h, sizeof(double) * h->slot_M[0]);
-        memcpy(h->frames.h + (size_t)i * N * kFrameStride, h->frames.h, sizeof(double) * N * kFrameStride);
         h->perm[i] = h->perm[0]; h->perm_identity[i] = h->perm_identity[0]; h->slot_M[i] = h->slot_M[0]; h->slot_N[i] = h->slot_N[0]; h->slot_K[i] = h->slot_K[0];
-        if (h->have_inertial) {
-            const size_t dcap = 15 * N;
-            memcpy(h->imu_idx.h + (size_t)i * N * 2, h->imu_idx.h, sizeof(int32_t) * N * 2);
-            memcpy(h->imu_data.h + (size_t)i * N * kImuStride, h->imu_data.h, sizeof(double) * N * kImuStride);
-            memcpy(h->prior_frames.h + (size_t)i * N, h->prior_frames.h, sizeof(int32_t) * N);
-            memcpy(h->prior_S.h + (size_t)i * dcap * dcap, h->prior_S.h, sizeof(double) * dcap * dcap);
-            memcpy(h->prior_e.h + (size_t)i * dcap, h->prior_e.h, sizeof(double) * dcap);
-            memcpy(h->prior_x0.h + (size_t)i * N * kFrameStride, h->prior_x0.h, sizeof(double) * N * kFrameStride);
-        }
-        if (h->have_planes) {
-            memcpy(h->plane_param.h + (size_t)i * h->Pcap * 4, h->plane_param.h, sizeof(double) * h->Pcap * 4);
-            memcpy(h->pt_plane.h + (size_t)i * h->Tcap, h->pt_plane.h, sizeof(int32_t) * h->Tcap);
-            memcpy(h->pt_begin.h + (size_t)i * (h->Tcap + 1), h->pt_begin.h, sizeof(int32_t) * (h->Tcap + 1));
-            memcpy(h->pt_frame.h + (size_t)i * h->Ocap, h->pt_frame.h, sizeof(int32_t) * h->Ocap);
-            memcpy(h->pt_z.h + (size_t)i * h->Ocap * 2, h->pt_z.h, sizeof(float) * h->Ocap * 2);
-        }
     }
     return 0;
 }
@@ -1065,96 +1155,18 @@ int pvio_b200_batch_download(pvio_b200_handle hh, int n, double *dx, int64_t dx_
     return download_dx(h, n, dx, dx_stride, costs);
 }
 
-// sub-batch schedule of the pipelined host paths: small batches first and last (the first upload and the last
-// kernels + download are the only parts of the pipeline that nothing overlaps), 512-window batches in between
-#ifndef PVIO_PIPE_STREAMS
-#define PVIO_PIPE_STREAMS 6
-#endif
-#ifndef PVIO_PIPE_CHUNK
-#define PVIO_PIPE_CHUNK 512
-#endif
-static constexpr int kPipeStreams = PVIO_PIPE_STREAMS;   // sub-batches in flight on the SMs at once (each alone is latency-bound: one wave)
-static std::vector<int> sub_batches(int n) {
-    std::vector<int> sizes;
-    if (n < 1024) { sizes.push_back(n); return sizes; }
-    int mid = n - 2 * (128 + 256);
-    sizes.push_back(128); sizes.push_back(256);
-    while (mid > 0) { const int m = std::min(PVIO_PIPE_CHUNK, mid); sizes.push_back(m); mid -= m; }
-    sizes.push_back(256); sizes.push_back(128);
-    return sizes;
-}
-
-static int ensure_pipeline_streams(Handle *h, int nsub) {
-    if (!h->stream_up) {
-        CK(h, cudaStreamCreateWithFlags(&h->stream_up, cudaStreamNonBlocking));
-        CK(h, cudaStreamCreateWithFlags(&h->stream_down, cudaStreamNonBlocking));
-    }
-    while ((int)h->ev_up.size() < nsub) {
-        cudaEvent_t a, b, c_;
-        CK(h, cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
-        CK(h, cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
-        CK(h, cudaEventCreateWithFlags(&c_, cudaEventDisableTiming));
-        h->ev_up.push_back(a); h->ev_done.push_back(b); h->ev_down.push_back(c_);
-    }
-    if (h->stream_c.empty()) {
-        h->stream_c.resize(kPipeStreams);
-        for (auto &st : h->stream_c) CK(h, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-        CK(h, cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-    }
-    return 0;
-}
-
-// End-to-end step with HOST buffers.  Large batches are cut into sub-batches and pipelined over
-// three streams: host->device copy of sub-batch i+1 overlaps the kernels of sub-batch i and the
-// device->host copy of sub-batch i-1 (PCIe is full duplex), so the call costs
-// max(copy, compute) instead of their sum.
+// End-to-end Gauss-Newton step with HOST buffers (run_pipelined).
 int pvio_b200_batch_gn_step_host(pvio_b200_handle hh, int n, double mu, double *dx, int64_t dx_stride, double *costs) {
     Handle *h = reinterpret_cast<Handle *>(hh);
     if (!h) return PVIO_B200_EINVAL;
-    if (n < 1 || n > h->W) return fail(h, PVIO_B200_EINVAL, "bad window count");
-    const std::vector<int> sizes = sub_batches(n);
-    const int nsub = (int)sizes.size();
-    if (nsub == 1) {
-        TRY(upload(h, n));
-        StepCfg c;
-        c.mu = mu; c.apply = 0; c.compute_scale = 1;
-        TRY(run_gn_step(h, n, c, batch_shape(h, 0, n, false)));
-        return download_dx(h, n, dx, dx_stride, costs);
-    }
-    std::vector<int> starts(nsub, 0);
-    for (int i = 1; i < nsub; ++i) starts[i] = starts[i - 1] + sizes[i - 1];
-    TRY(ensure_pipeline_streams(h, nsub));
-    CK(h, cudaEventRecord(h->ev_fork, h->stream));
-    CK(h, cudaStreamWaitEvent(h->stream_up, h->ev_fork, 0));
-    for (auto &sc : h->stream_c) CK(h, cudaStreamWaitEvent(sc, h->ev_fork, 0));
-    for (int i = 0; i < nsub; ++i) {
-        const int w0 = starts[i], m = sizes[i];
-        cudaStream_t sc = h->stream_c[i % kPipeStreams];
-        TRY(upload_range(h, w0, m, h->stream_up));
-        CK(h, cudaEventRecord(h->ev_up[i], h->stream_up));
-        CK(h, cudaStreamWaitEvent(sc, h->ev_up[i], 0));
-        StepCfg c;
-        c.mu = mu; c.apply = 0; c.compute_scale = 1; c.w0 = w0; c.stream = sc;
-        TRY(run_gn_step(h, m, c, batch_shape(h, w0, m, false)));
-        CK(h, cudaEventRecord(h->ev_done[i], sc));
-        CK(h, cudaStreamWaitEvent(h->stream_down, h->ev_done[i], 0));
-        CK(h, cudaStreamWaitEvent(h->stream, h->ev_done[i], 0));
-        CK(h, cudaMemcpyAsync(h->dx_pose.h + (size_t)w0 * h->Ncap * 15, h->dx_pose.d + (size_t)w0 * h->Ncap * 15,
-                              sizeof(double) * h->Ncap * 15 * m, cudaMemcpyDeviceToHost, h->stream_down));
-        CK(h, cudaMemcpyAsync(h->dx_lm.h + (size_t)w0 * h->Mcap, h->dx_lm.d + (size_t)w0 * h->Mcap,
-                              sizeof(double) * h->Mcap * m, cudaMemcpyDeviceToHost, h->stream_down));
-        CK(h, cudaMemcpyAsync(h->ctrl.h + w0, h->ctrl.d + w0, sizeof(WinCtrl) * m, cudaMemcpyDeviceToHost, h->stream_down));
-        CK(h, cudaEventRecord(h->ev_down[i], h->stream_down));
-    }
-    h->n_uploaded = n;
-    // scatter each sub-batch as soon as it has landed, while the GPU works on the later ones
-    for (int i = 0; i < nsub; ++i) {
-        const int w0 = starts[i], m = sizes[i];
-        CK(h, cudaEventSynchronize(h->ev_down[i]));
-        TRY(scatter_dx(h, w0, m, dx, dx_stride, costs));
-    }
-    CK(h, cudaStreamSynchronize(h->stream));
-    return 0;
+    return run_pipelined(h, n,
+        [&](int w0, int m, cudaStream_t st) {
+            StepCfg c;
+            c.mu = mu; c.apply = 0; c.compute_scale = 1; c.w0 = w0; c.stream = st;
+            return run_gn_step(h, m, c, batch_shape(h, w0, m, false));
+        },
+        [&](int w0, int m, cudaStream_t st) { return download_dx_async(h, w0, m, st); },
+        [&](int w0, int m) { return scatter_dx(h, w0, m, dx, dx_stride, costs); });
 }
 
 // Full trust-region solve (device-side loop, per-window termination) of the first n uploaded windows; the states on
@@ -1163,9 +1175,7 @@ int pvio_b200_batch_solve(pvio_b200_handle hh, int n, const pvio_b200_options *o
     Handle *h = reinterpret_cast<Handle *>(hh);
     if (!h) return PVIO_B200_EINVAL;
     if (n < 1 || n > h->n_uploaded) return fail(h, PVIO_B200_EINVAL, "windows not uploaded");
-    const int max_iter = opt ? opt->max_iterations : 10;
-    const double radius0 = (opt && opt->initial_trust_region_radius > 0) ? opt->initial_trust_region_radius : 1e4;
-    return run_solve_loop(h, n, max_iter, opt ? opt->max_time : 0.0, radius0, opt ? opt->alias_bias : 1);
+    return run_solve_loop(h, 0, n, h->stream, solve_opts(opt));
 }
 
 int pvio_b200_batch_download_state(pvio_b200_handle hh, int n, double *frames, int64_t frames_stride, double *inv_depth,
@@ -1175,76 +1185,24 @@ int pvio_b200_batch_download_state(pvio_b200_handle hh, int n, double *frames, i
     if (n < 1 || n > h->W) return fail(h, PVIO_B200_EINVAL, "bad window count");
     TRY(download_state_async(h, 0, n, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    for (int i = 0; i < n; ++i) {
-        scatter_state(h, i, frames ? frames + (size_t)i * frames_stride : nullptr, inv_depth ? inv_depth + (size_t)i * inv_depth_stride : nullptr);
-        if (summaries) fill_summary(h->ctrl.h[i], &summaries[i]);
-    }
+    scatter_states(h, 0, n, frames, frames_stride, inv_depth, inv_depth_stride, summaries);
     return 0;
 }
 
-// upload + solve + download with HOST buffers, pipelined over sub-batches like pvio_b200_batch_gn_step_host: one
-// host -> device copy buys up to max_iterations Gauss-Newton iterations per window.
+// upload + solve + download with HOST buffers (run_pipelined): one host -> device copy buys up to max_iterations
+// Gauss-Newton iterations per window.
 int pvio_b200_batch_solve_host(pvio_b200_handle hh, int n, const pvio_b200_options *opt, double *frames, int64_t frames_stride,
                                double *inv_depth, int64_t inv_depth_stride, pvio_b200_summary *summaries) {
     Handle *h = reinterpret_cast<Handle *>(hh);
     if (!h) return PVIO_B200_EINVAL;
-    if (n < 1 || n > h->W) return fail(h, PVIO_B200_EINVAL, "bad window count");
-    const int max_iter = opt ? opt->max_iterations : 10;
-    const double radius0 = (opt && opt->initial_trust_region_radius > 0) ? opt->initial_trust_region_radius : 1e4;
-    const int alias = opt ? opt->alias_bias : 1;
-    const std::vector<int> sizes = sub_batches(n);
-    const int nsub = (int)sizes.size();
-    if (nsub == 1) {
-        TRY(upload(h, n));
-        TRY(run_solve_loop(h, n, max_iter, opt ? opt->max_time : 0.0, radius0, alias));
-        return pvio_b200_batch_download_state(hh, n, frames, frames_stride, inv_depth, inv_depth_stride, summaries);
-    }
-    std::vector<int> starts(nsub, 0);
-    for (int i = 1; i < nsub; ++i) starts[i] = starts[i - 1] + sizes[i - 1];
-    TRY(ensure_pipeline_streams(h, nsub));
-#ifdef PVIO_TUNE_TIMING
-    const auto tt0 = std::chrono::steady_clock::now();
-    auto stamp = [&](const char *what) { fprintf(stderr, "  [%s] %.3f ms\n", what, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tt0).count()); };
-#else
-    auto stamp = [&](const char *) {};
-#endif
-    // sub-batch i: upload on the copy stream, the whole trust-region loop on compute stream i % kPipeStreams (a sub-batch
-    // is at most one wave of CTAs, so alone it runs at the latency of its kernel chain; several in flight fill the SMs),
-    // download on the second copy stream; the windows of different sub-batches share nothing on the device
-    CK(h, cudaEventRecord(h->ev_fork, h->stream));
-    CK(h, cudaStreamWaitEvent(h->stream_up, h->ev_fork, 0));
-    for (auto &sc : h->stream_c) CK(h, cudaStreamWaitEvent(sc, h->ev_fork, 0));
-    for (int i = 0; i < nsub; ++i) {
-        const int w0 = starts[i], m = sizes[i];
-        cudaStream_t sc = h->stream_c[i % kPipeStreams];
-        TRY(upload_range(h, w0, m, h->stream_up));
-        CK(h, cudaEventRecord(h->ev_up[i], h->stream_up));
-        CK(h, cudaStreamWaitEvent(sc, h->ev_up[i], 0));
-        StepCfg c;
-        c.mu = -1.0; c.loop = 1; c.alias_bias = alias; c.compute_scale = 0; c.w0 = w0; c.stream = sc;
-        const BatchShape b = batch_shape(h, w0, m, false);
-        init_ctrl_kernel<<<m, 32, 0, sc>>>(h->ctrl.d, 1e-8, radius0, max_iter, opt ? opt->max_time : 0.0, w0);
-        ++h->launches;
-        for (int it = 0; it < max_iter + 2; ++it) TRY(iteration_body(h, m, c, b, it == 0));
-        CK(h, cudaEventRecord(h->ev_done[i], sc));
-        CK(h, cudaStreamWaitEvent(h->stream_down, h->ev_done[i], 0));
-        CK(h, cudaStreamWaitEvent(h->stream, h->ev_done[i], 0));      // later calls on the handle's stream see the result
-        TRY(download_state_async(h, w0, m, h->stream_down));
-        CK(h, cudaEventRecord(h->ev_down[i], h->stream_down));
-    }
-    h->n_uploaded = n;
-    stamp("enqueued");
-    for (int i = 0; i < nsub; ++i) {
-        CK(h, cudaEventSynchronize(h->ev_down[i]));
-        stamp("sub-batch landed");
-        for (int k = starts[i]; k < starts[i] + sizes[i]; ++k) {
-            scatter_state(h, k, frames ? frames + (size_t)k * frames_stride : nullptr, inv_depth ? inv_depth + (size_t)k * inv_depth_stride : nullptr);
-            if (summaries) fill_summary(h->ctrl.h[k], &summaries[k]);
-        }
-    }
-    CK(h, cudaStreamSynchronize(h->stream));
-    stamp("done");
-    return 0;
+    const SolveOpts o = solve_opts(opt);
+    return run_pipelined(h, n,
+        [&](int w0, int m, cudaStream_t st) { return run_solve_loop(h, w0, m, st, o); },
+        [&](int w0, int m, cudaStream_t st) { return download_state_async(h, w0, m, st); },
+        [&](int w0, int m) {
+            scatter_states(h, w0, m, frames, frames_stride, inv_depth, inv_depth_stride, summaries);
+            return 0;
+        });
 }
 
 int pvio_b200_ba_gn_step(pvio_b200_handle hh, const pvio_b200_window *w, const pvio_b200_state *s, double mu,
@@ -1282,13 +1240,10 @@ int pvio_b200_ba_solve(pvio_b200_handle hh, const pvio_b200_window *w, pvio_b200
                        const pvio_b200_options *opt, pvio_b200_summary *summary, uint8_t *valid, double *quality) {
     Handle *h = reinterpret_cast<Handle *>(hh);
     if (!h || !w || !s) return PVIO_B200_EINVAL;
-    const int max_iter = opt ? opt->max_iterations : 10;
-    const int alias = opt ? opt->alias_bias : 1;
-    const double radius0 = (opt && opt->initial_trust_region_radius > 0) ? opt->initial_trust_region_radius : 1e4;
     TRY(pack_window(h, 0, w, s));
     TRY(upload(h, 1));
     CK(h, cudaEventRecord(h->ev0, h->stream));
-    TRY(run_solve_loop(h, 1, max_iter, opt ? opt->max_time : 0.0, radius0, alias));
+    TRY(run_solve_loop(h, 0, 1, h->stream, solve_opts(opt)));
     CK(h, cudaEventRecord(h->ev1, h->stream));
     const int M = w->n_landmarks;
     const bool post = (!opt || opt->run_postpass) && (valid || quality);
@@ -1299,7 +1254,7 @@ int pvio_b200_ba_solve(pvio_b200_handle hh, const pvio_b200_window *w, pvio_b200
     }
     TRY(download_state_async(h, 0, 1, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    scatter_state(h, 0, s->frames, s->inv_depth);
+    scatter_states(h, 0, 1, s->frames, 0, s->inv_depth, 0, summary);
     if (post) {
         const std::vector<int32_t> &perm = h->perm[0];
         for (int lp = 0; lp < M; ++lp) {
@@ -1308,7 +1263,6 @@ int pvio_b200_ba_solve(pvio_b200_handle hh, const pvio_b200_window *w, pvio_b200
         }
     }
     if (summary) {
-        fill_summary(h->ctrl.h[0], summary);
         float ms = 0.f;
         cudaEventElapsedTime(&ms, h->ev0, h->ev1);
         summary->solve_seconds = ms * 1e-3;

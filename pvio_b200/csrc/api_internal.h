@@ -5,17 +5,29 @@
 #include <map>
 #include <string>
 #include <tuple>
+#include <utility>
 #include <vector>
 #include "../../include/pvio_b200.h"
 #include "ba_types.h"
 
 namespace pvio {
 
+// Owns a device array and its optional pinned host staging; both are freed with the buffer.
 template <typename T>
 struct DevBuf {
     T *d = nullptr;      // device
     T *h = nullptr;      // pinned host staging (optional)
     size_t n = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    DevBuf(DevBuf &&o) noexcept { swap(o); }
+    DevBuf &operator=(DevBuf &&o) noexcept { DevBuf(std::move(o)).swap(*this); return *this; }
+    ~DevBuf() {
+        if (d) cudaFree(d);
+        if (h) cudaFreeHost(h);
+    }
+    void swap(DevBuf &o) noexcept { std::swap(d, o.d); std::swap(h, o.h); std::swap(n, o.n); }
 };
 
 struct KltState;         // klt.cu
@@ -60,7 +72,8 @@ struct Handle {
     DevBuf<int32_t> lm_msk;                      // [W][Mcap] frame mask of each landmark
     bool hs_double = false;
     DevBuf<double> frames_out, rho_out;          // pinned landing area of downloaded states (the upload staging stays intact)
-    DevBuf<double> Hred, Hdd, gdir, gred, cost_vis, acc, aux_cost;
+    DevBuf<double> Hred, acc, aux_cost;
+    double *Hdd = nullptr, *gdir = nullptr, *gred = nullptr, *cost_vis = nullptr;   // views into the Hred allocation
     DevBuf<double> Hfull, gfull;                 // debug dump (single window only)
     DevBuf<uint8_t> valid;                       // post-pass results
     DevBuf<double> quality;
@@ -96,6 +109,15 @@ struct Handle {
 };
 
 int fail(Handle *h, int code, const char *what, cudaError_t e = cudaSuccess);
+
+// pvio_b200_options with its defaults filled in (opt may be NULL)
+struct SolveOpts {
+    int max_iter = 10;
+    double radius0 = 1e4;
+    int alias_bias = 1;
+    double max_time = 0.0;
+};
+SolveOpts solve_opts(const pvio_b200_options *opt);
 
 #define CK(h, call)                                                        \
     do {                                                                   \

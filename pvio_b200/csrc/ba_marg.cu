@@ -481,7 +481,7 @@ int marginalize_impl(Handle *h, const pvio_b200_window *w, const pvio_b200_state
     rc = run_marg_vision(h);
     if (rc != 0) return rc;
     MargArgs m;
-    m.hdr = h->hdr.d; m.cst = h->cst.d; m.frames = h->frames.d; m.Hred = h->Hred.d; m.gred = h->gred.d;
+    m.hdr = h->hdr.d; m.cst = h->cst.d; m.frames = h->frames.d; m.Hred = h->Hred.d; m.gred = h->gred;
     m.imu_idx = h->imu_idx.d; m.imu_data = h->imu_data.d; m.prior_frames = h->prior_frames.d;
     m.prior_S = h->prior_S.d; m.prior_L = h->prior_L.d; m.prior_e = h->prior_e.d; m.prior_x0 = h->prior_x0.d;
     m.Ncap = h->Ncap; m.index = index; m.H = dH; m.b = db; m.scratch = dscr;

@@ -307,8 +307,9 @@ int pnp_solve_impl(Handle *h, const pvio_b200_pnp_problem *pb, double *frame, co
     memset(&a, 0, sizeof(a));
     a.pts = d; a.z = d + 3 * n; a.frame = d + 5 * n; a.out = d + 5 * n + 16; a.imu_rec = d + 5 * n + 24;
     a.n = n; a.inertial = pb->use_inertial ? 1 : 0;
-    a.max_iter = opt ? opt->max_iterations : 10;
-    a.radius0 = (opt && opt->initial_trust_region_radius > 0) ? opt->initial_trust_region_radius : 1e4;
+    const SolveOpts o = solve_opts(opt);
+    a.max_iter = o.max_iter;
+    a.radius0 = o.radius0;
     memcpy(a.wc.cam_q, pb->cam_q_cs, 32); memcpy(a.wc.cam_p, pb->cam_p_cs, 24);
     memcpy(a.wc.imu_q, pb->imu_q_cs, 32); memcpy(a.wc.imu_p, pb->imu_p_cs, 24);
     memcpy(a.wc.sic, pb->sqrt_inv_cov, 32);

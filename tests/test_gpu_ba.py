@@ -204,6 +204,24 @@ def test_throughput_heterogeneous_batch(mixed_inertial):
             assert abs(costs[i, 0] - ref['cost']) <= 2e-6 * ref['cost']
 
 
+def test_plane_buffers_grow_without_losing_packed_slots():
+    """A window with more plane tracks than the plane arrays hold makes them grow while slot 0 is packed: slot 0's
+    plane tracks must survive the move to the larger per-window stride."""
+    small = synth.make_cfg4(N=6, M=60, tracks_per_plane=20)[:2]
+    large = synth.make_cfg4(N=6, M=60, tracks_per_plane=150, seed=651)[:2]
+    assert large[0].n_ptracks > 256
+    b = BundleAdjustor(max_windows=2, max_frames=6, max_landmarks=64, max_obs=400)
+    b.batch_set(0, *small)
+    b.batch_set(1, *large)
+    b.batch_upload(2)
+    b.batch_gn_step(2, 1e-8, apply=False)
+    dx, _ = b.batch_download(2, 15 * 6 + 64)
+    b.close()
+    for i, (w, st) in enumerate((small, large)):
+        ref = bo.gn_step(w, st, schur=True)
+        assert _rel(dx[i, :15 * w.N + w.M], ref['dx']) < TOL_DX, i
+
+
 def test_full_size_batch_properties():
     """BASELINE's full bench size (4096 cfg2 windows per launch): size-independent properties instead of 4096 oracle
     runs -- replicas are bit-identical, the second half of the batch is scaled noise (different data) and must still
@@ -348,6 +366,28 @@ def test_pipelined_host_step_matches_resident_step():
     b.close()
 
 
+def test_pipelined_host_solve_matches_resident_solve():
+    """pvio_b200_batch_solve_host over >= 1024 windows runs the trust-region solve sub-batch by sub-batch; every window
+    must end where batch_upload + batch_solve + batch_download_state takes it.  The inertial kind sends the IMU and
+    prior arrays through the pipelined upload."""
+    W, N, M = 1100, 6, 64
+    kinds = [synth.make_cfg2(N=6, M=48, seed=910)[:2], synth.make_cfg2(N=5, M=40, seed=911)[:2],
+             synth.make_cfg2(N=6, M=48, staggered=True, seed=912)[:2], synth.make_cfg3(N=6, M=60, seed=913)[:2]]
+    b = BundleAdjustor(max_windows=W, max_frames=N, max_landmarks=M, max_obs=400)
+    for i in range(W):
+        b.batch_set(i, *kinds[i % len(kinds)])
+    frames_h, rho_h, sm_h = b.batch_solve_host(W, N, M, max_iterations=8)
+    b.batch_upload(W)
+    b.batch_solve(W, max_iterations=8)
+    frames_d, rho_d, sm_d = b.batch_download_state(W, N, M)
+    b.close()
+    for i in range(W):
+        for k in ('iterations', 'accepted_steps', 'termination'):
+            assert getattr(sm_h[i], k) == sm_d[i][k], (i, k)
+    assert np.allclose(frames_h.reshape(W, N, 16), frames_d, rtol=0, atol=1e-9)
+    assert np.allclose(rho_h[:, :M], rho_d, rtol=1e-9, atol=0)
+
+
 # ------------------------------------------------------------------ golden vectors and edge cases
 import os as _os
 _GOLD = _os.path.join(_os.path.dirname(_os.path.abspath(__file__)), "golden", "ba_golden.npz")
@@ -470,6 +510,25 @@ def test_batch_solve_matches_single_window_solve(ba):
         assert np.allclose(frames[i, :w.N, 4:7], ref_state.p, rtol=0, atol=1e-9)
         assert np.allclose(rho[i, :w.M], ref_state.rho, rtol=1e-9, atol=0)
     assert len({sm[i]['iterations'] for i in range(3)}) > 1        # the windows really stopped at different iterations
+
+
+def test_host_solve_single_sub_batch_matches_single_window_solve(ba):
+    """pvio_b200_batch_solve_host below the pipelining threshold: one upload, solve and download on the handle's
+    stream; every window gets the result of its own pvio_b200_ba_solve."""
+    kinds = [synth.make_cfg2(N=6, M=80, seed=54)[:2], synth.make_cfg2(N=5, M=40, seed=55)[:2],
+             synth.make_cfg2(N=6, M=80, staggered=True, seed=56)[:2]]
+    singles = [ba.solve(w, st, max_iterations=7) for w, st in kinds]
+    for i, (w, st) in enumerate(kinds):
+        ba.batch_set(i, w, st)
+    frames, rho, sm = ba.batch_solve_host(3, 6, 80, max_iterations=7)
+    frames = frames.reshape(3, 6, 16)
+    for i, (w, st) in enumerate(kinds):
+        ref_state, ref_sum = singles[i]
+        assert sm[i].iterations == ref_sum['iterations'] and sm[i].termination == ref_sum['termination']
+        assert sm[i].accepted_steps == ref_sum['accepted_steps']
+        assert abs(sm[i].final_cost - ref_sum['final_cost']) <= 1e-9 * ref_sum['final_cost']
+        assert np.allclose(frames[i, :w.N, 4:7], ref_state.p, rtol=0, atol=1e-9)
+        assert np.allclose(rho[i, :w.M], ref_state.rho, rtol=1e-9, atol=0)
 
 
 def test_device_lie_group_helpers_across_taylor_branches(ba):

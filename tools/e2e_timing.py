@@ -1,5 +1,5 @@
 """Tuning aid: wall time of the pipelined end-to-end solve (pvio_b200_batch_solve_host) for a library variant
-named by PVIO_B200_TUNE_LIB (built with -DPVIO_TUNE_TIMING it also prints the sub-batch landing times)."""
+named by PVIO_B200_TUNE_LIB."""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
